@@ -8,6 +8,7 @@ configuration the metric is quoted on and fits one GPU.  A step = one drain of t
 whole batch.  "samples" = sum over streams of post-resample, pre-mix samples (SURVEY.md §8d).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
+  python bench.py ... --dump-outputs DIR                        # also writes the last timed step's mix to DIR/mix.npy
   python bench.py --impl reference ...                          # the reference's CPU algorithm (oracle port,
                                                                 # all host threads; rodio is Rust and cannot be built here)
 Under torchrun (N>1) every rank renders its own 4096 streams (weak scaling), the partial mixes are
@@ -31,6 +32,7 @@ sys.path.insert(0, ROOT)
 
 MIX_CH, MIX_RATE, IN_RATE = 1, 48000, 44100
 LOW_PASS_HZ, AMPLIFY = 200, 1.2
+DUMP_MAX_SAMPLES = 1 << 23      # 32 MB of float32: a longer mix is dumped as a fixed, seeded sample of its samples
 
 
 def parse():
@@ -44,7 +46,14 @@ def parse():
     ap.add_argument("--flags", type=int, default=0, help="rb_batch_create flags (debug)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the mix of the last timed step to DIR/mix.npy (float32), for comparing two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def measured_traffic(workload: str, streams: int, seconds: float):
@@ -96,6 +105,7 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()
         sm = [float(r[0]) for r in self.rows if len(r) >= 6 and r[0].replace(".", "").isdigit()]
         mx = [float(r[1]) for r in self.rows if len(r) >= 6 and r[1].replace(".", "").isdigit()]
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
@@ -170,10 +180,8 @@ def run_reference(args):
     n_streams = args.streams
     streams = cpu_streams(n_streams, frames)
     cpu_reference(streams[:max(1, min(n_streams, threads))], frames, threads)          # warm-up (page in, spawn)
-    first = cpu_reference(streams, frames, threads)
-    # the whole run stays within about two minutes: as many of the requested steps as fit
-    steps = max(3, min(args.steps, int(90.0 / max(first[1], 1e-3))))
-    runs = [first] + [cpu_reference(streams, frames, threads) for _ in range(steps - 1)]
+    steps = args.steps
+    runs = [cpu_reference(streams, frames, threads) for _ in range(steps)]
     vals = sorted(r[0] for r in runs)
     value = statistics.median(vals)
     secs_all = sum(r[1] for r in runs)
@@ -248,7 +256,9 @@ def run_ours(args):
     gen = torch.Generator(device=dev)
     gen.manual_seed(0x5EED + rank)
     with torch.cuda.stream(ext):
-        arena.uniform_(-1.0, 1.0, generator=gen)
+        # drawn as a packed (streams, frames) block and copied into the batch's pitched rows: the same seed gives every stream
+        # the same samples whatever padding the library puts between streams
+        arena.as_strided((S, frames), (pitch, 1)).copy_(torch.empty(S, frames, device=dev).uniform_(-1.0, 1.0, generator=gen))
     mix = torch.as_tensor(rbd.DeviceArray(batch.mix_device_ptr, max(1, mix_len)), device=dev)
 
     def step():
@@ -274,6 +284,8 @@ def run_ours(args):
         step()
     e1.record(ext)
     fence()
+    # what the last timed step handed its caller, copied before the loops below render into the same buffer
+    last_mix = mix[:mix_len].cpu().numpy() if args.dump_outputs else None
     ms_total = e0.elapsed_time(e1)
     ms_total = rbd.max_over_ranks(ms_total, dev)
     ms_step = ms_total / args.steps
@@ -545,6 +557,11 @@ def run_ours(args):
             "gpu_launches": launches * args.steps,
             "clocks": clocks,
         }
+        if args.dump_outputs:
+            if last_mix.size > DUMP_MAX_SAMPLES:
+                last_mix = last_mix[np.sort(np.random.default_rng(0).choice(last_mix.size, DUMP_MAX_SAMPLES, replace=False))]
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "mix.npy"), last_mix)
         print(json.dumps(line), flush=True)
     batch.close()
     if world > 1:
